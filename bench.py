@@ -5,6 +5,7 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W   (N > 1, one rank per GPU)
   python bench.py --impl reference --gpus 1 --steps 3 --warmup 1  (reference arm: oracle port on host cores)
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR  (also writes the last step's outputs as .npy)
 
 A "step" = one pass of the hot path over one build context per GPU:
   CRC-32 context fingerprint (cacheID, bit-exact reference arithmetic) + Roll-32 CDC + per-chunk SHA-256
@@ -73,7 +74,44 @@ def parse():
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-deliverables", action="store_true", help="skip the {cacheID, TarDigest} same-deliverables leg")
     ap.add_argument("--deliv-one-layer-mib", type=int, default=256, help="sample size of the ONE-layer TarDigest run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last device-resident step computed to DIR/<name>.npy "
+                         "(single-process runs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_ROWS = 65536  # chunk-table rows kept by --dump-outputs: a seeded sample when the table is longer (about 18 MB in all)
+
+
+def dump_outputs(eng, res, out_dir: str):
+    """What a caller of the device-resident path receives from one step, as float64 / float32 arrays (every value is
+    exact in them): the result struct, the context CRC-32 (cacheID), and the same seeded sample of rows of the chunk
+    list (end offset + SHA-256) and of the sorted unique-digest table."""
+    os.makedirs(out_dir, exist_ok=True)
+    n_chunks, n_unique = int(res.n_chunks), int(res.n_unique)
+    ends, digs = eng.get_chunks(n_chunks)
+    table = eng.get_table(n_unique)
+
+    def rows(n):
+        if n <= DUMP_ROWS:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    ci, ti = rows(n_chunks), rows(n_unique)
+    arrays = {
+        "result_counts": np.array([res.crc_bytes, res.cdc_bytes, res.n_files, n_chunks, n_unique], dtype=np.float64),
+        "cache_id_crc32": np.array([eng.ctx_crc32(res)], dtype=np.float64),
+        "merkle_root": np.frombuffer(bytes(res.root), dtype=np.uint8).astype(np.float32),
+        "chunk_rows": ci.astype(np.float64),
+        "chunk_ends": ends[ci].astype(np.float64),
+        "chunk_sha256": digs[ci].astype(np.float32),
+        "table_rows": ti.astype(np.float64),
+        "table_sha256": table[ti].astype(np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -610,6 +648,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs is for single-process runs (the chunk list of a rank is not the exchanged table's)")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; the B200 path has no CPU fallback")
     torch.cuda.set_device(local)
@@ -761,6 +801,8 @@ def main():
     st1 = eng.stats()
     dt = max_over_ranks(dt)
     launches = int(st1.kernel_launches - st0.kernel_launches)
+    if args.dump_outputs:
+        dump_outputs(eng, res, args.dump_outputs)
     ms_step = dt / args.steps * 1e3
     ctx_bytes = lay["data_bytes"]
     value = world * ctx_bytes / GiB / (dt / args.steps)
@@ -846,7 +888,7 @@ def main():
         s0 = eng2.stats()
         barrier()
         t0 = time.perf_counter()
-        n_e2e = max(2, min(args.steps, 3))
+        n_e2e = args.steps
         for _ in range(n_e2e):
             r = e2e_step()
         barrier()
@@ -1012,7 +1054,7 @@ def main():
                 sstep()
             barrier()
             t0 = time.perf_counter()
-            n_s = max(2, args.steps)
+            n_s = args.steps
             for _ in range(n_s):
                 sr = sstep()
             barrier()

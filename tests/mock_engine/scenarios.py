@@ -475,12 +475,13 @@ def ingest_member_larger_than_the_arena(make_engine, tmp):
               "small.txt": b"hello"}
     buf = io.BytesIO()
     with tarfile.open(fileobj=buf, mode="w", format=tarfile.PAX_FORMAT) as tf:
+        # members owned by the caller: the untar below must reach the capacity check, not fail on chown
         d = tarfile.TarInfo("big/")
-        d.type, d.mode, d.mtime = tarfile.DIRTYPE, 0o755, T
+        d.type, d.mode, d.mtime, d.uid, d.gid = tarfile.DIRTYPE, 0o755, T, os.getuid(), os.getgid()
         tf.addfile(d)
         for name, data in bodies.items():
             ti = tarfile.TarInfo(name)
-            ti.size, ti.mode, ti.mtime = len(data), 0o644, T
+            ti.size, ti.mode, ti.mtime, ti.uid, ti.gid = len(data), 0o644, T, os.getuid(), os.getgid()
             tf.addfile(ti, io.BytesIO(data))
     data = buf.getvalue()
     path = os.path.join(tmp, "big.tar")

@@ -145,7 +145,9 @@ def test_layer_and_on_disk_copy_agree_on_symlinked_sources(tmp_path, linked_ctx)
     files -- they disagreed while only Execute resolved its sources."""
     dst_root = tmp_path / "fsroot"
     dst_root.mkdir()
-    host.copy_op_execute(host.CopyOperation(["/linkdir"], linked_ctx, "/", str(dst_root / "dst")))
+    # --chown to the caller (without it the copy is owned by 0:0), so the copy needs no privilege
+    host.copy_op_execute(host.CopyOperation(["/linkdir"], linked_ctx, "/", str(dst_root / "dst"), os.getuid(), os.getgid()),
+                         host.MKHOST_COPY_CHOWN)
     on_disk = sorted(os.path.relpath(os.path.join(d, f), dst_root) for d, ds, fs in os.walk(dst_root) for f in fs + ds)
     ents = _layer_both(tmp_path, linked_ctx, ["/linkdir"], "/dst")
     assert on_disk == sorted(e[1].lstrip("/") for e in ents)

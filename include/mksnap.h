@@ -230,6 +230,38 @@ uint64_t mksnap_table_rows(mksnap_t *h);
  * lib/builder/step/common.go:86 (hex-encode and prefix "sha256:" on the host). */
 int mksnap_get_stream_digests(mksnap_t *h, uint8_t *digests, uint64_t capacity);
 
+/* ---- chunk index and chunk delta (DESIGN.md section 3b) ----
+ * A chunk index is a sorted-unique set of 32-byte chunk digests that lives in HBM and outlives sessions (the layers a
+ * registry or cache already holds).  Rows are ordered bytewise over all 32 bytes -- the order of mksnap_get_table --
+ * and mksnap_index_get returns that order, so an index persists as get -> store anywhere -> add_rows.
+ * An index works with any handle on the device it was created on (another device: MKSNAP_E_INVAL).  add_rows and
+ * add_table return MKSNAP_E_CAPACITY only when the UNION would exceed capacity_rows; on any error the index is
+ * unchanged.  add_rows checks strict ascent on the device (violation: MKSNAP_E_INVAL).
+ * mksnap_delta, add_table and get_chunk_status need a finished session whose table is still its own: before finish,
+ * after the next begin, on one rank of several, or after an exchange / all-gather they return MKSNAP_E_STATE.
+ * Per layer: finish -> delta(ix) -> add_table(ix).  The delta classifies against the index as it is at call time;
+ * statuses stay valid until the next begin. */
+typedef struct mksnap_index mksnap_index_t;
+int mksnap_index_create(mksnap_t *h, uint64_t capacity_rows, mksnap_index_t **out); /* on h's device; capacity < 2^32 */
+void mksnap_index_destroy(mksnap_index_t *ix);                                        /* before the handle it was created on */
+uint64_t mksnap_index_rows(const mksnap_index_t *ix);
+int mksnap_index_add_rows(mksnap_t *h, mksnap_index_t *ix, const uint8_t *rows, uint64_t n); /* host rows, strictly ascending */
+int mksnap_index_add_table(mksnap_t *h, mksnap_index_t *ix);      /* union with h's finished session table */
+int mksnap_index_get(mksnap_t *h, mksnap_index_t *ix, uint8_t *rows, uint64_t capacity_rows);
+
+#define MKSNAP_CHUNK_KNOWN 0u  /* digest is in the index */
+#define MKSNAP_CHUNK_NEW 1u    /* not in the index; lowest chunk position carrying this digest in the session */
+#define MKSNAP_CHUNK_REPEAT 2u /* not in the index; an earlier chunk of the session has the same digest */
+typedef struct {
+    uint64_t index_rows;
+    uint64_t known_chunks, new_chunks, repeat_chunks;
+    uint64_t known_bytes, new_bytes, repeat_bytes; /* sum to mksnap_result.cdc_bytes */
+    float ms_device;                               /* CUDA events around the delta's kernels */
+    uint32_t reserved;
+} mksnap_delta_result;
+int mksnap_delta(mksnap_t *h, const mksnap_index_t *ix, mksnap_delta_result *out); /* after mksnap_finish */
+int mksnap_get_chunk_status(mksnap_t *h, uint8_t *status, uint64_t capacity);      /* one byte per chunk, mksnap_get_chunks order */
+
 /* ---- multi-GPU: one process per GPU, files sharded, one exchange step ---- */
 /* NCCL is dlopen()ed (libnccl.so.2); rank 0 creates the id, the host side
  * distributes it (any out-of-band channel), every rank calls comm_init. */

@@ -323,3 +323,108 @@ func (e *Engine) ContextCRC32Cached(cc *CrcCache, prefix []byte, contextDir stri
 	}
 	return uint32(c), uint64(st.bytes_sent), nil
 }
+
+// Index is a device-resident sorted-unique set of chunk digests (mksnap_index_*): the chunks of the base image and of
+// the layers already pushed or cached.  It lives on the engine's device and outlives sessions; Close it before the
+// engine it was created on.
+type Index struct {
+	ix *C.mksnap_index_t
+	e  *Engine
+}
+
+// NewIndex creates an empty index of capacityRows rows (< 2^32) on e's device.
+func (e *Engine) NewIndex(capacityRows uint64) (*Index, error) {
+	x := &Index{e: e}
+	if rc := C.mksnap_index_create(e.h, C.uint64_t(capacityRows), &x.ix); rc != 0 {
+		return nil, fmt.Errorf("mksnap index create: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	return x, nil
+}
+
+// Close releases the index's device memory.
+func (x *Index) Close() {
+	if x.ix != nil {
+		C.mksnap_index_destroy(x.ix)
+		x.ix = nil
+	}
+}
+
+// Rows is the number of digests the index holds.
+func (x *Index) Rows() uint64 { return uint64(C.mksnap_index_rows(x.ix)) }
+
+// AddTable adds the chunk table of e's finished session (base-layer ingest or a committed layer).
+func (x *Index) AddTable(e *Engine) error {
+	if rc := C.mksnap_index_add_table(e.h, x.ix); rc != 0 {
+		return fmt.Errorf("mksnap index add table: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	return nil
+}
+
+// AddRows adds persisted rows: n*32 bytes, strictly ascending (what Rows returned, stored anywhere).
+func (x *Index) AddRows(rows []byte) error {
+	if len(rows)%32 != 0 {
+		return fmt.Errorf("mksnap index add rows: %d bytes is not a multiple of 32", len(rows))
+	}
+	if len(rows) == 0 {
+		return nil
+	}
+	p := C.CBytes(rows)
+	defer C.free(p)
+	if rc := C.mksnap_index_add_rows(x.e.h, x.ix, (*C.uint8_t)(p), C.uint64_t(len(rows)/32)); rc != 0 {
+		return fmt.Errorf("mksnap index add rows: %s", C.GoString(C.mksnap_last_error(x.e.h)))
+	}
+	return nil
+}
+
+// Get returns the index rows in bytewise order, 32 bytes each: the persisted form of the index.
+func (x *Index) Get() ([]byte, error) {
+	n := x.Rows()
+	if n == 0 {
+		return nil, nil
+	}
+	buf := C.malloc(C.size_t(n * 32))
+	defer C.free(buf)
+	if rc := C.mksnap_index_get(x.e.h, x.ix, (*C.uint8_t)(buf), C.uint64_t(n)); rc != 0 {
+		return nil, fmt.Errorf("mksnap index get: %s", C.GoString(C.mksnap_last_error(x.e.h)))
+	}
+	return C.GoBytes(buf, C.int(n*32)), nil
+}
+
+// Chunk statuses of Delta / ChunkStatus.
+const (
+	ChunkKnown  = 0 // the digest is in the index
+	ChunkNew    = 1 // not in the index; the first chunk of the layer carrying it
+	ChunkRepeat = 2 // not in the index; an earlier chunk of the layer has the same digest
+)
+
+// DeltaResult counts the chunks and bytes of each status.  NewBytes is what a chunk-granular push would send.
+type DeltaResult struct {
+	IndexRows                            uint64
+	KnownChunks, NewChunks, RepeatChunks uint64
+	KnownBytes, NewBytes, RepeatBytes    uint64
+	DeviceMs                             float32
+}
+
+// Delta classifies every chunk of e's finished session against x.  Call it before x.AddTable(e) for the same layer.
+func (e *Engine) Delta(x *Index) (DeltaResult, error) {
+	var r C.mksnap_delta_result
+	if rc := C.mksnap_delta(e.h, x.ix, &r); rc != 0 {
+		return DeltaResult{}, fmt.Errorf("mksnap delta: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	return DeltaResult{IndexRows: uint64(r.index_rows), KnownChunks: uint64(r.known_chunks), NewChunks: uint64(r.new_chunks),
+		RepeatChunks: uint64(r.repeat_chunks), KnownBytes: uint64(r.known_bytes), NewBytes: uint64(r.new_bytes),
+		RepeatBytes: uint64(r.repeat_bytes), DeviceMs: float32(r.ms_device)}, nil
+}
+
+// ChunkStatus returns one status byte per chunk of the last Delta, in chunk order (valid until the next session).
+func (e *Engine) ChunkStatus(nChunks uint64) ([]byte, error) {
+	if nChunks == 0 {
+		return nil, nil
+	}
+	buf := C.malloc(C.size_t(nChunks))
+	defer C.free(buf)
+	if rc := C.mksnap_get_chunk_status(e.h, (*C.uint8_t)(buf), C.uint64_t(nChunks)); rc != 0 {
+		return nil, fmt.Errorf("mksnap chunk status: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	return C.GoBytes(buf, C.int(nChunks)), nil
+}

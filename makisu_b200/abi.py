@@ -70,6 +70,17 @@ class Limits(C.Structure):
                 ("n_device_slots", C.c_uint32), ("carry_bytes", C.c_uint64)]
 
 
+MKSNAP_CHUNK_KNOWN = 0   # digest is in the index
+MKSNAP_CHUNK_NEW = 1     # not in the index; lowest chunk position carrying this digest in the session
+MKSNAP_CHUNK_REPEAT = 2  # not in the index; an earlier chunk of the session has the same digest
+
+
+class DeltaResult(C.Structure):
+    _fields_ = [("index_rows", C.c_uint64), ("known_chunks", C.c_uint64), ("new_chunks", C.c_uint64),
+                ("repeat_chunks", C.c_uint64), ("known_bytes", C.c_uint64), ("new_bytes", C.c_uint64),
+                ("repeat_bytes", C.c_uint64), ("ms_device", C.c_float), ("reserved", C.c_uint32)]
+
+
 # every symbol include/mksnap.h declares: (name, restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = [
@@ -93,6 +104,14 @@ SYMBOLS = [
     ("mksnap_get_chunks", C.c_int, [_P, _P, _P, C.c_uint64]),
     ("mksnap_get_table", C.c_int, [_P, _P, C.c_uint64]),
     ("mksnap_get_stream_digests", C.c_int, [_P, _P, C.c_uint64]),
+    ("mksnap_index_create", C.c_int, [_P, C.c_uint64, C.POINTER(_P)]),
+    ("mksnap_index_destroy", None, [_P]),
+    ("mksnap_index_rows", C.c_uint64, [_P]),
+    ("mksnap_index_add_rows", C.c_int, [_P, _P, _P, C.c_uint64]),
+    ("mksnap_index_add_table", C.c_int, [_P, _P]),
+    ("mksnap_index_get", C.c_int, [_P, _P, _P, C.c_uint64]),
+    ("mksnap_delta", C.c_int, [_P, _P, C.POINTER(DeltaResult)]),
+    ("mksnap_get_chunk_status", C.c_int, [_P, _P, C.c_uint64]),
     ("mksnap_comm_unique_id", C.c_int, [_P]),
     ("mksnap_comm_init", C.c_int, [_P, _P, C.c_int32, C.c_int32]),
     ("mksnap_table_rows", C.c_uint64, [_P]),
@@ -284,6 +303,20 @@ class Engine:
         self._ck(self.lib.mksnap_stats(self.h, C.byref(s)), "mksnap_stats")
         return s
 
+    # -- chunk delta ---------------------------------------------------
+    def delta(self, ix: "ChunkIndex") -> DeltaResult:
+        """Classify every chunk of the finished session against `ix` (MKSNAP_CHUNK_KNOWN / NEW / REPEAT)."""
+        r = DeltaResult()
+        self._ck(self.lib.mksnap_delta(self.h, ix.ix, C.byref(r)), "mksnap_delta")
+        return r
+
+    def chunk_status(self, n: int):
+        """The statuses of the last delta, one uint8 per chunk in get_chunks order."""
+        import numpy as np
+        out = np.empty(max(n, 1), dtype=np.uint8)
+        self._ck(self.lib.mksnap_get_chunk_status(self.h, out.ctypes.data, n), "mksnap_get_chunk_status")
+        return out[:n]
+
     # -- multi GPU -----------------------------------------------------
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -319,6 +352,49 @@ class Engine:
             msgs = [(e.lib.mksnap_last_error(e.h) or b"").decode() for e in engines]
             raise MksnapError(rc, "mksnap_exchange_tables_local", "; ".join(m for m in msgs if m))
         return [outs[i] for i in range(n)]
+
+
+class ChunkIndex:
+    """A device-resident sorted-unique set of chunk digests (mksnap_index_*), created on `eng`'s device.  Every call
+    takes an engine on that device; close() before the engine it was created on is closed."""
+
+    def __init__(self, eng: Engine, capacity_rows: int):
+        self.lib = eng.lib
+        self.capacity = capacity_rows
+        self.ix = _P()
+        eng._ck(self.lib.mksnap_index_create(eng.h, capacity_rows, C.byref(self.ix)), "mksnap_index_create")
+
+    def rows(self) -> int:
+        return int(self.lib.mksnap_index_rows(self.ix))
+
+    def add_rows(self, eng: Engine, rows):
+        """Union with host rows: an (n, 32) uint8 array, strictly ascending bytewise."""
+        import numpy as np
+        a = np.ascontiguousarray(rows, dtype=np.uint8).reshape(-1, 32)
+        eng._ck(self.lib.mksnap_index_add_rows(eng.h, self.ix, a.ctypes.data if a.size else None, a.shape[0]),
+                "mksnap_index_add_rows")
+
+    def add_table(self, eng: Engine):
+        """Union with eng's finished session table."""
+        eng._ck(self.lib.mksnap_index_add_table(eng.h, self.ix), "mksnap_index_add_table")
+
+    def get(self, eng: Engine):
+        import numpy as np
+        n = self.rows()
+        out = np.empty((max(n, 1), 32), dtype=np.uint8)
+        eng._ck(self.lib.mksnap_index_get(eng.h, self.ix, out.ctypes.data, n), "mksnap_index_get")
+        return out[:n]
+
+    def close(self):
+        if getattr(self, "ix", None):
+            self.lib.mksnap_index_destroy(self.ix)
+            self.ix = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
 
 
 def exchange_plan(rows_per_rank, rank: int) -> dict:

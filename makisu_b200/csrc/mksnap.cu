@@ -5,6 +5,7 @@
 // mksnap_kernels.cuh; there is deliberately no CPU fallback.
 #include "../../include/mksnap.h"
 #include "mksnap_kernels.cuh"
+#include "mksnap_index.cuh"
 
 #include <dlfcn.h>
 #include <stdarg.h>
@@ -139,7 +140,17 @@ struct mksnap {
     uint8_t root[32];
     bool finished = false;
     bool in_session = false;
+    bool table_own = false; // d_table is the finished session's own table (set by finish; cleared by begin, exchange, all-gather)
     mksnap_result last_result;
+
+    // chunk delta: allocated by the first mksnap_delta, sized for max_chunks
+    uint32_t *d_dfirst = nullptr; // per session-table row: lowest non-known chunk carrying it
+    uint32_t *d_duidx = nullptr;  // per chunk: its session-table row (IDX_NONE = known)
+    uint32_t *d_ddir = nullptr;   // prefix directory of d_table
+    uint8_t *d_dstatus = nullptr; // per chunk: MKSNAP_CHUNK_*
+    unsigned long long *d_dcnt = nullptr;
+    cudaEvent_t ev_delta[2] = {nullptr, nullptr};
+    bool delta_done = false; // d_dstatus holds this session's statuses
 
     // multi-GPU
     NcclApi nccl;
@@ -226,9 +237,15 @@ void build_crc_consts(CrcConsts *c)
     }
 }
 
-// generic device exclusive scan (u32), in -> out (may alias), n elements
-int scan_u32(mksnap *h, const uint32_t *in, uint32_t *out, uint64_t n, cudaStream_t s)
+// generic device exclusive scan (u32), in -> out (may alias), n elements; block sums go to h->d_scan_tmp unless the
+// caller brings its own temporary
+int scan_u32(mksnap *h, const uint32_t *in, uint32_t *out, uint64_t n, cudaStream_t s, uint32_t *tmp = nullptr,
+             uint64_t tmp_words = 0)
 {
+    if (!tmp) {
+        tmp = h->d_scan_tmp;
+        tmp_words = h->scan_tmp_words;
+    }
     if (n == 0)
         return 0;
     // level sizes
@@ -243,21 +260,21 @@ int scan_u32(mksnap *h, const uint32_t *in, uint32_t *out, uint64_t n, cudaStrea
         off[l] = total;
         total += sizes[l];
     }
-    if (total > h->scan_tmp_words)
+    if (total > tmp_words)
         return fail(h, MKSNAP_E_CAPACITY, "scan temp too small (%llu > %llu)", (unsigned long long)total,
-                    (unsigned long long)h->scan_tmp_words);
+                    (unsigned long long)tmp_words);
     // up-sweep: reduce each level into the next
     for (size_t l = 0; l + 1 < sizes.size(); l++) {
-        const uint32_t *src = l == 0 ? in : h->d_scan_tmp + off[l];
+        const uint32_t *src = l == 0 ? in : tmp + off[l];
         uint32_t nb = (uint32_t)sizes[l + 1];
-        k_scan_reduce<<<nb, 256, 0, s>>>(src, sizes[l], h->d_scan_tmp + off[l + 1]);
+        k_scan_reduce<<<nb, 256, 0, s>>>(src, sizes[l], tmp + off[l + 1]);
         LAUNCH_OK(h);
     }
     // top level fits one block: scan in place
     for (size_t l = sizes.size(); l-- > 0;) {
-        const uint32_t *src = l == 0 ? in : h->d_scan_tmp + off[l];
-        uint32_t *dst = l == 0 ? out : h->d_scan_tmp + off[l];
-        const uint32_t *boff = (l + 1 < sizes.size()) ? h->d_scan_tmp + off[l + 1] : nullptr;
+        const uint32_t *src = l == 0 ? in : tmp + off[l];
+        uint32_t *dst = l == 0 ? out : tmp + off[l];
+        const uint32_t *boff = (l + 1 < sizes.size()) ? tmp + off[l + 1] : nullptr;
         uint32_t nb = (uint32_t)((sizes[l] + SCAN_ITEMS - 1) / SCAN_ITEMS);
         k_scan_apply<<<nb, 256, 0, s>>>(src, sizes[l], boff, dst);
         LAUNCH_OK(h);
@@ -674,6 +691,10 @@ void mksnap_destroy(mksnap_t *h)
     cudaFree(h->d_sorted); cudaFree(h->d_table); cudaFree(h->d_flags); cudaFree(h->d_pos); cudaFree(h->d_hist);
     cudaFree(h->d_gather); cudaFree(h->d_gcount); cudaFree(h->d_concat);
     cudaFree(h->d_xbounds); cudaFree(h->d_xhdr); cudaFree(h->d_xrec); cudaFree(h->d_xtail);
+    cudaFree(h->d_dfirst); cudaFree(h->d_duidx); cudaFree(h->d_ddir); cudaFree(h->d_dstatus); cudaFree(h->d_dcnt);
+    for (int i = 0; i < 2; i++)
+        if (h->ev_delta[i])
+            cudaEventDestroy(h->ev_delta[i]);
     if (h->s_comp) cudaStreamDestroy(h->s_comp);
     if (h->s_copy) cudaStreamDestroy(h->s_copy);
     delete h;
@@ -698,6 +719,8 @@ int mksnap_begin(mksnap_t *h)
     h->open_file = false;
     h->n_unique = 0;
     h->finished = false;
+    h->table_own = false;
+    h->delta_done = false;
     h->in_session = true;
     return 0;
 }
@@ -1135,6 +1158,7 @@ int mksnap_finish(mksnap_t *h, mksnap_result *out)
     out->n_streams = h->n_streams;
     h->last_result = *out;
     h->finished = true;
+    h->table_own = h->n_ranks == 1;
     return 0;
 }
 
@@ -1253,6 +1277,277 @@ int mksnap_stats(mksnap_t *h, mksnap_stats_t *out)
     *out = h->stats;
     return 0;
 }
+// ---- chunk index and chunk delta (DESIGN.md section 3b) ---------------------------------------------------------
+struct mksnap_index {
+    int device = 0;
+    uint64_t cap = 0, n = 0;
+    uint32_t bits = 0;                 // directory bits of the current table
+    int cur = 0;                       // rows[cur] / dir[cur] hold the index; the other pair is the spare a union builds
+    uint8_t *rows[2] = {nullptr, nullptr};
+    uint32_t *dir[2] = {nullptr, nullptr};
+    uint8_t *novel = nullptr;          // compacted rows a union adds
+    uint8_t *stage = nullptr;          // uploaded rows of add_rows (allocated by the first add_rows)
+    uint32_t *flags = nullptr, *pos = nullptr, *scan_tmp = nullptr;
+    uint64_t scan_words = 0;
+    uint32_t *d_bad = nullptr;
+};
+
+static mk::RowSet index_view(const mksnap_index *ix)
+{
+    return mk::RowSet{ix->rows[ix->cur], ix->dir[ix->cur], (uint32_t)ix->n, ix->bits};
+}
+
+static uint32_t grid_for(uint64_t n, uint32_t tb) { return (uint32_t)std::max<uint64_t>(1, (n + tb - 1) / tb); }
+
+// delta / add_table / get_chunk_status need the finished session's own table on a single-rank handle
+static int own_table_check(mksnap *h, const mksnap_index *ix, const char *what)
+{
+    if (ix && ix->device != h->cfg.device)
+        return fail(h, MKSNAP_E_INVAL, "%s: index lives on device %d, handle on device %d", what, ix->device, h->cfg.device);
+    if (!h->finished)
+        return fail(h, MKSNAP_E_STATE, "%s needs a finished session", what);
+    if (h->n_ranks > 1)
+        return fail(h, MKSNAP_E_STATE, "%s: the handle is one rank of %d (its table is a shard)", what, h->n_ranks);
+    if (!h->table_own)
+        return fail(h, MKSNAP_E_STATE, "%s: an exchange or all-gather replaced the session's table", what);
+    return 0;
+}
+
+static void index_free(mksnap_index *ix)
+{
+    for (int k = 0; k < 2; k++) {
+        cudaFree(ix->rows[k]);
+        cudaFree(ix->dir[k]);
+    }
+    cudaFree(ix->novel); cudaFree(ix->stage); cudaFree(ix->flags); cudaFree(ix->pos); cudaFree(ix->scan_tmp); cudaFree(ix->d_bad);
+    delete ix;
+}
+
+int mksnap_index_create(mksnap_t *h, uint64_t capacity_rows, mksnap_index_t **out)
+{
+    if (!h || !out)
+        return MKSNAP_E_INVAL;
+    *out = nullptr;
+    if (capacity_rows >= (1ull << 32))
+        return fail(h, MKSNAP_E_INVAL, "index capacity %llu rows: must be below 2^32", (unsigned long long)capacity_rows);
+    CK(h, cudaSetDevice(h->cfg.device));
+    mksnap_index *ix = new mksnap_index;
+    ix->device = h->cfg.device;
+    ix->cap = capacity_rows;
+    const uint64_t rows = std::max<uint64_t>(1, capacity_rows);
+    const uint64_t dir_words = (1ull << mk::dir_bits(capacity_rows)) + 1;
+    ix->scan_words = rows / SCAN_ITEMS * 2 + 4096;
+    cudaError_t e = cudaSuccess;
+    for (int k = 0; k < 2 && e == cudaSuccess; k++) {
+        e = cudaMalloc(&ix->rows[k], rows * 32);
+        if (e == cudaSuccess)
+            e = cudaMalloc(&ix->dir[k], dir_words * 4);
+    }
+    if (e == cudaSuccess) e = cudaMalloc(&ix->novel, rows * 32);
+    if (e == cudaSuccess) e = cudaMalloc(&ix->flags, rows * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&ix->pos, rows * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&ix->scan_tmp, ix->scan_words * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&ix->d_bad, 4);
+    if (e == cudaSuccess) {
+        k_dir_build<<<1, 256, 0, h->s_comp>>>(ix->rows[0], 0, 0, ix->dir[0]); // the empty index: dir = {0, 0}
+        e = cudaGetLastError();
+        if (e == cudaSuccess)
+            e = cudaStreamSynchronize(h->s_comp);
+    }
+    if (e != cudaSuccess) {
+        index_free(ix);
+        return fail(h, e == cudaErrorMemoryAllocation ? MKSNAP_E_NOMEM : MKSNAP_E_CUDA, "mksnap_index_create: %s",
+                    cudaGetErrorString(e));
+    }
+    h->stats.kernel_launches++;
+    *out = ix;
+    return 0;
+}
+
+void mksnap_index_destroy(mksnap_index_t *ix)
+{
+    if (!ix)
+        return;
+    cudaSetDevice(ix->device);
+    index_free(ix);
+}
+
+uint64_t mksnap_index_rows(const mksnap_index_t *ix) { return ix ? ix->n : 0; }
+
+// index := index U src[0, m) (src sorted-unique, on the device).  Novel rows = rows the index lookup misses, compacted
+// with scan_u32; the merge writes into the spare buffer and the pair is swapped only when everything succeeded.
+static int index_union(mksnap *h, mksnap_index *ix, const uint8_t *src, uint64_t m, bool check_ascent)
+{
+    if (m > ix->cap) // m distinct rows: the union holds at least m
+        return fail(h, MKSNAP_E_CAPACITY, "%llu incoming rows exceed the index capacity %llu", (unsigned long long)m,
+                    (unsigned long long)ix->cap);
+    cudaStream_t s = h->s_comp;
+    if (check_ascent) {
+        CK(h, cudaMemsetAsync(ix->d_bad, 0, 4, s));
+        if (m > 1) {
+            k_check_ascent<<<grid_for(m - 1, 256), 256, 0, s>>>(src, (uint32_t)m, ix->d_bad);
+            LAUNCH_OK(h);
+        }
+    }
+    k_novel_flags<<<grid_for(m, 256), 256, 0, s>>>(src, (uint32_t)m, index_view(ix), ix->flags);
+    LAUNCH_OK(h);
+    int rc = scan_u32(h, ix->flags, ix->pos, m, s, ix->scan_tmp, ix->scan_words);
+    if (rc)
+        return rc;
+    uint32_t tail[3] = {0, 0, 0}; // last pos, last flag, ascent violated
+    CK(h, cudaMemcpyAsync(&tail[0], ix->pos + (m - 1), 4, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaMemcpyAsync(&tail[1], ix->flags + (m - 1), 4, cudaMemcpyDeviceToHost, s));
+    if (check_ascent)
+        CK(h, cudaMemcpyAsync(&tail[2], ix->d_bad, 4, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s));
+    h->stats.d2h_bytes += check_ascent ? 12 : 8;
+    if (tail[2])
+        return fail(h, MKSNAP_E_INVAL, "index_add_rows: rows are not strictly ascending");
+    const uint64_t novel = (uint64_t)tail[0] + tail[1];
+    if (ix->n + novel > ix->cap)
+        return fail(h, MKSNAP_E_CAPACITY, "union of %llu index rows and %llu new rows exceeds capacity %llu",
+                    (unsigned long long)ix->n, (unsigned long long)novel, (unsigned long long)ix->cap);
+    if (novel == 0)
+        return 0;
+    k_compact_digests<<<grid_for(2 * m, 256), 256, 0, s>>>(src, ix->flags, ix->pos, m, ix->novel);
+    LAUNCH_OK(h);
+    const int nxt = ix->cur ^ 1;
+    const uint64_t total = ix->n + novel;
+    k_merge_rows<<<grid_for(total, MERGE_TILE), MERGE_THREADS, 0, s>>>(ix->rows[ix->cur], (uint32_t)ix->n, ix->novel,
+                                                                      (uint32_t)novel, ix->rows[nxt]);
+    LAUNCH_OK(h);
+    const uint32_t bits = mk::dir_bits(total);
+    k_dir_build<<<grid_for(total + 1, 256), 256, 0, s>>>(ix->rows[nxt], (uint32_t)total, bits, ix->dir[nxt]);
+    LAUNCH_OK(h);
+    CK(h, cudaStreamSynchronize(s));
+    ix->cur = nxt;
+    ix->n = total;
+    ix->bits = bits;
+    return 0;
+}
+
+int mksnap_index_add_rows(mksnap_t *h, mksnap_index_t *ix, const uint8_t *rows, uint64_t n)
+{
+    if (!h || !ix || (n && !rows))
+        return MKSNAP_E_INVAL;
+    if (ix->device != h->cfg.device)
+        return fail(h, MKSNAP_E_INVAL, "index_add_rows: index lives on device %d, handle on device %d", ix->device, h->cfg.device);
+    if (n == 0)
+        return 0;
+    if (n > ix->cap) // before the upload: the staging buffer holds capacity rows
+        return fail(h, MKSNAP_E_CAPACITY, "index_add_rows: %llu rows exceed capacity %llu", (unsigned long long)n,
+                    (unsigned long long)ix->cap);
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (!ix->stage)
+        CK(h, cudaMalloc(&ix->stage, std::max<uint64_t>(1, ix->cap) * 32));
+    // on the compute stream: a pageable cudaMemcpy may return before its DMA lands, and nothing would order the
+    // kernels that read the rows after it
+    CK(h, cudaMemcpyAsync(ix->stage, rows, n * 32, cudaMemcpyHostToDevice, h->s_comp));
+    h->stats.h2d_bytes += n * 32;
+    return index_union(h, ix, ix->stage, n, true);
+}
+
+int mksnap_index_add_table(mksnap_t *h, mksnap_index_t *ix)
+{
+    if (!h || !ix)
+        return MKSNAP_E_INVAL;
+    int rc = own_table_check(h, ix, "index_add_table");
+    if (rc)
+        return rc;
+    CK(h, cudaSetDevice(h->cfg.device));
+    return h->n_unique ? index_union(h, ix, h->d_table, h->n_unique, false) : 0;
+}
+
+int mksnap_index_get(mksnap_t *h, mksnap_index_t *ix, uint8_t *rows, uint64_t capacity_rows)
+{
+    if (!h || !ix || (ix->n && !rows))
+        return MKSNAP_E_INVAL;
+    if (ix->device != h->cfg.device)
+        return fail(h, MKSNAP_E_INVAL, "index_get: index lives on device %d, handle on device %d", ix->device, h->cfg.device);
+    if (ix->n > capacity_rows)
+        return fail(h, MKSNAP_E_CAPACITY, "index_get: need %llu rows", (unsigned long long)ix->n);
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (ix->n) {
+        CK(h, cudaStreamSynchronize(h->s_comp));
+        CK(h, cudaMemcpy(rows, ix->rows[ix->cur], ix->n * 32, cudaMemcpyDeviceToHost));
+    }
+    h->stats.d2h_bytes += ix->n * 32;
+    return 0;
+}
+
+int mksnap_delta(mksnap_t *h, const mksnap_index_t *ix, mksnap_delta_result *out)
+{
+    if (!h || !ix || !out)
+        return MKSNAP_E_INVAL;
+    int rc = own_table_check(h, ix, "delta");
+    if (rc)
+        return rc;
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (!h->d_dstatus) { // first use: the delta's buffers, sized for the session
+        const uint64_t mc = std::max<uint64_t>(1, h->max_chunks);
+        CK(h, cudaMalloc(&h->d_dfirst, mc * 4));
+        CK(h, cudaMalloc(&h->d_duidx, mc * 4));
+        CK(h, cudaMalloc(&h->d_ddir, ((1ull << mk::dir_bits(mc)) + 1) * 4));
+        CK(h, cudaMalloc(&h->d_dcnt, 6 * sizeof(unsigned long long)));
+        CK(h, cudaMalloc(&h->d_dstatus, mc));
+        for (int i = 0; i < 2; i++)
+            CK(h, cudaEventCreate(&h->ev_delta[i]));
+    }
+    cudaStream_t s = h->s_comp;
+    const uint64_t n = h->last_result.n_chunks, u = h->n_unique;
+    CK(h, cudaEventRecord(h->ev_delta[0], s));
+    CK(h, cudaMemsetAsync(h->d_dcnt, 0, 6 * sizeof(unsigned long long), s));
+    if (n) {
+        CK(h, cudaMemsetAsync(h->d_dfirst, 0xFF, u * 4, s));
+        const uint32_t tbits = mk::dir_bits(u);
+        k_dir_build<<<grid_for(u + 1, 256), 256, 0, s>>>(h->d_table, (uint32_t)u, tbits, h->d_ddir);
+        LAUNCH_OK(h);
+        k_delta_lookup<<<grid_for(n, 256), 256, 0, s>>>(h->d_digests, (uint32_t)n, index_view(ix),
+                                                        mk::RowSet{h->d_table, h->d_ddir, (uint32_t)u, tbits}, h->d_dstatus,
+                                                        h->d_duidx, h->d_dfirst);
+        LAUNCH_OK(h);
+        const uint32_t grid = (uint32_t)std::min<uint64_t>(grid_for(n, DELTA_THREADS), (uint64_t)h->sm_count * 8);
+        k_delta_classify<<<grid, DELTA_THREADS, 0, s>>>((uint32_t)n, h->d_duidx, h->d_dfirst, h->d_chunk_len, h->d_dstatus,
+                                                        h->d_dcnt);
+        LAUNCH_OK(h);
+    }
+    CK(h, cudaEventRecord(h->ev_delta[1], s));
+    unsigned long long c[6];
+    CK(h, cudaMemcpyAsync(c, h->d_dcnt, sizeof c, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s));
+    h->stats.d2h_bytes += sizeof c;
+    memset(out, 0, sizeof *out);
+    out->index_rows = ix->n;
+    out->known_chunks = c[0];
+    out->new_chunks = c[1];
+    out->repeat_chunks = c[2];
+    out->known_bytes = c[3];
+    out->new_bytes = c[4];
+    out->repeat_bytes = c[5];
+    CK(h, cudaEventElapsedTime(&out->ms_device, h->ev_delta[0], h->ev_delta[1]));
+    h->delta_done = true;
+    return 0;
+}
+
+int mksnap_get_chunk_status(mksnap_t *h, uint8_t *status, uint64_t capacity)
+{
+    if (!h)
+        return MKSNAP_E_INVAL;
+    int rc = own_table_check(h, nullptr, "get_chunk_status");
+    if (rc)
+        return rc;
+    if (!h->delta_done)
+        return fail(h, MKSNAP_E_STATE, "get_chunk_status before mksnap_delta in this session");
+    const uint64_t n = h->last_result.n_chunks;
+    if (n > capacity || (n && !status))
+        return fail(h, MKSNAP_E_CAPACITY, "need %llu bytes", (unsigned long long)n);
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (n)
+        CK(h, cudaMemcpy(status, h->d_dstatus, n, cudaMemcpyDeviceToHost));
+    h->stats.d2h_bytes += n;
+    return 0;
+}
+
 #include "mksnap_comm.inc"
 
 } // extern "C"

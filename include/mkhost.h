@@ -145,7 +145,11 @@ int mkhost_memfs_commit_scan(mkhost_memfs *m, mksnap_t *eng, int64_t now_unix, i
  * The reference commits layer by layer (build_node.go:102-107); COPY/ADD steps that do not modify the file system
  * (no RUN in between) can be deferred and committed together, which is what a cgo caller would do (INTEGRATION.md).
  * outs[i].tar_digest / tar_bytes / n_entries are per layer; root / n_chunks / n_unique describe the chunk table of the
- * whole batch (one session).  flags: MKHOST_NO_TAR_DIGEST only.  tar_fd < 0: that layer's tar is not emitted. */
+ * whole batch (one session) -- unless MKHOST_LAYER_TABLES is set: then the session is grouped (layer i = group i,
+ * mksnap_begin_groups) and they are layer i's own, equal to what a separate mkhost_memfs_commit_copy_ops of that layer
+ * returns; the engine's session stays open for mksnap_delta_groups / mksnap_get_group_table / mksnap_index_add_group.
+ * flags: MKHOST_NO_TAR_DIGEST, MKHOST_LAYER_TABLES.  tar_fd < 0: that layer's tar is not emitted. */
+#define MKHOST_LAYER_TABLES 64u
 typedef struct {
     const mkhost_copy_op *ops;
     size_t n_ops;

@@ -262,6 +262,37 @@ typedef struct {
 int mksnap_delta(mksnap_t *h, const mksnap_index_t *ix, mksnap_delta_result *out); /* after mksnap_finish */
 int mksnap_get_chunk_status(mksnap_t *h, uint8_t *status, uint64_t capacity);      /* one byte per chunk, mksnap_get_chunks order */
 
+/* ---- grouped sessions: per-layer chunk tables and deltas in one session (DESIGN.md section 3c) ----
+ * mksnap_begin_groups starts a session whose every submit tags each extent with a group (1 <= n_groups <= 65536):
+ * consecutive layers committed together, layer i = group i.  The tag counts only on MKSNAP_X_CDC extents, must be
+ * < n_groups, and the pieces of one split file (MKSNAP_X_MORE / MKSNAP_X_CONT) carry the same group; otherwise the submit
+ * returns MKSNAP_E_INVAL and the session is unchanged.  Everything the batch returns (mksnap_result, get_chunks,
+ * get_table, the root, mksnap_delta, index_add_table) is byte-identical to the same submits in an ungrouped session.
+ * Finish also builds, per group, the sorted-unique table and root (and n_files, cdc_bytes, n_chunks, n_unique) that an
+ * ungrouped session of only that group's CDC extents, in the same order, would return.  A plain submit in a grouped
+ * session, a grouped submit or any getter below in an ungrouped one, and begin_groups on one rank of several return
+ * MKSNAP_E_STATE.  Group results stay valid until the next begin. */
+int mksnap_begin_groups(mksnap_t *h, uint32_t n_groups);
+int mksnap_arena_submit_groups(mksnap_t *h, int32_t arena_id, uint64_t used, const mksnap_extent *extents,
+                               uint64_t n_extents, const uint32_t *groups /* one per extent */,
+                               const mksnap_range *ranges, uint64_t n_ranges);
+int mksnap_device_submit_groups(mksnap_t *h, uint32_t slot, uint64_t used, const mksnap_extent *extents,
+                                uint64_t n_extents, const uint32_t *groups, const mksnap_range *ranges, uint64_t n_ranges);
+typedef struct {
+    uint64_t n_files, cdc_bytes, n_chunks, n_unique;
+    uint64_t first_row; /* where the group's table starts in the concatenation of all group tables */
+    uint8_t root[32];   /* fan-out-256 Merkle root of the group's table = the layer's content address */
+} mksnap_group_result;
+int mksnap_get_group_results(mksnap_t *h, mksnap_group_result *out, uint32_t n_groups); /* after finish; n_groups of the session */
+int mksnap_get_group_table(mksnap_t *h, uint32_t group, uint8_t *rows, uint64_t capacity_rows);
+int mksnap_get_chunk_groups(mksnap_t *h, uint32_t *groups, uint64_t capacity);           /* one per chunk, get_chunks order */
+/* The sequential per-layer flow "for g in 0..n-1: delta(ix) of layer g -> index_add_table(ix)" in one call, without
+ * changing ix: a chunk of group g is KNOWN if its digest is in ix or occurs in a group < g, NEW at the lowest position
+ * of group g carrying the digest, REPEAT otherwise.  out[g] gets group g's counts (index_rows = ix at call time);
+ * mksnap_get_chunk_status then returns these statuses. */
+int mksnap_delta_groups(mksnap_t *h, const mksnap_index_t *ix, mksnap_delta_result *out, uint32_t n_groups);
+int mksnap_index_add_group(mksnap_t *h, mksnap_index_t *ix, uint32_t group); /* union with one group's table */
+
 /* ---- multi-GPU: one process per GPU, files sharded, one exchange step ---- */
 /* NCCL is dlopen()ed (libnccl.so.2); rank 0 creates the id, the host side
  * distributes it (any out-of-band channel), every rank calls comm_init. */

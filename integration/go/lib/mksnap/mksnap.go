@@ -218,8 +218,14 @@ func (fs *MemFS) CommitScan(e *Engine, now int64, tarOut *os.File, threads int, 
 	return toResult(&r), nil
 }
 
+// LayerTables (flag of CommitLayers, MKHOST_LAYER_TABLES): give every layer of the batch its own chunk table -- ChunkRoot,
+// Chunks and Unique of result i are what CommitCopyOps of layer i alone returns -- and leave the grouped session open
+// for Engine.DeltaGroups / GroupTable / Index.AddGroup (layer i = group i).
+const LayerTables = 64
+
 // CommitLayers commits consecutive COPY/ADD layers of one build in ONE engine session: every TarDigest chain
 // advances together on the device (one chain runs at ~0.09 GB/s, 256 chains at ~23 GB/s).  tarOuts[i] may be nil.
+// Without LayerTables in flags, ChunkRoot / Chunks / Unique of every result describe the batch as a whole.
 func (fs *MemFS) CommitLayers(e *Engine, now int64, layers [][]CopyOp, tarOuts []*os.File, threads int, flags uint32) ([]LayerResult, error) {
 	n := len(layers)
 	specs := (*C.mkhost_layer_spec)(C.calloc(C.size_t(n+1), C.size_t(unsafe.Sizeof(C.mkhost_layer_spec{}))))
@@ -427,4 +433,76 @@ func (e *Engine) ChunkStatus(nChunks uint64) ([]byte, error) {
 		return nil, fmt.Errorf("mksnap chunk status: %s", C.GoString(C.mksnap_last_error(e.h)))
 	}
 	return C.GoBytes(buf, C.int(nChunks)), nil
+}
+
+// GroupResult is one group (layer) of a grouped session: its own chunk table, as if it had been committed alone.
+type GroupResult struct {
+	Files, CdcBytes, Chunks, Unique, FirstRow uint64
+	Root                                      [32]byte
+}
+
+// GroupResults returns the per-group results of e's finished grouped session (CommitLayers with LayerTables).
+func (e *Engine) GroupResults(nGroups int) ([]GroupResult, error) {
+	if nGroups <= 0 {
+		return nil, fmt.Errorf("mksnap group results: %d groups", nGroups)
+	}
+	buf := (*C.mksnap_group_result)(C.calloc(C.size_t(nGroups), C.size_t(unsafe.Sizeof(C.mksnap_group_result{}))))
+	defer C.free(unsafe.Pointer(buf))
+	if rc := C.mksnap_get_group_results(e.h, buf, C.uint32_t(nGroups)); rc != 0 {
+		return nil, fmt.Errorf("mksnap group results: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	view := (*[1 << 20]C.mksnap_group_result)(unsafe.Pointer(buf))[:nGroups:nGroups]
+	out := make([]GroupResult, nGroups)
+	for i := range out {
+		r := &view[i]
+		out[i] = GroupResult{Files: uint64(r.n_files), CdcBytes: uint64(r.cdc_bytes), Chunks: uint64(r.n_chunks),
+			Unique: uint64(r.n_unique), FirstRow: uint64(r.first_row)}
+		copy(out[i].Root[:], C.GoBytes(unsafe.Pointer(&r.root[0]), 32))
+	}
+	return out, nil
+}
+
+// GroupTable returns group g's sorted-unique chunk table (rows = its GroupResult.Unique), 32 bytes per row: the rows
+// to persist next to that layer's <key>_chunks entry.
+func (e *Engine) GroupTable(g int, rows uint64) ([]byte, error) {
+	if rows == 0 {
+		return nil, nil
+	}
+	buf := C.malloc(C.size_t(rows * 32))
+	defer C.free(buf)
+	if rc := C.mksnap_get_group_table(e.h, C.uint32_t(g), (*C.uint8_t)(buf), C.uint64_t(rows)); rc != 0 {
+		return nil, fmt.Errorf("mksnap group table: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	return C.GoBytes(buf, C.int(rows*32)), nil
+}
+
+// DeltaGroups is "for every layer g in order: Delta(x), then x.AddTable" over a grouped session in one call, without
+// changing x: a chunk of layer g is known if x holds it or an earlier layer of the batch has it.  ChunkStatus then
+// returns these statuses.
+func (e *Engine) DeltaGroups(x *Index, nGroups int) ([]DeltaResult, error) {
+	if nGroups <= 0 {
+		return nil, fmt.Errorf("mksnap delta groups: %d groups", nGroups)
+	}
+	buf := (*C.mksnap_delta_result)(C.calloc(C.size_t(nGroups), C.size_t(unsafe.Sizeof(C.mksnap_delta_result{}))))
+	defer C.free(unsafe.Pointer(buf))
+	if rc := C.mksnap_delta_groups(e.h, x.ix, buf, C.uint32_t(nGroups)); rc != 0 {
+		return nil, fmt.Errorf("mksnap delta groups: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	view := (*[1 << 20]C.mksnap_delta_result)(unsafe.Pointer(buf))[:nGroups:nGroups]
+	out := make([]DeltaResult, nGroups)
+	for i := range out {
+		r := &view[i]
+		out[i] = DeltaResult{IndexRows: uint64(r.index_rows), KnownChunks: uint64(r.known_chunks), NewChunks: uint64(r.new_chunks),
+			RepeatChunks: uint64(r.repeat_chunks), KnownBytes: uint64(r.known_bytes), NewBytes: uint64(r.new_bytes),
+			RepeatBytes: uint64(r.repeat_bytes), DeviceMs: float32(r.ms_device)}
+	}
+	return out, nil
+}
+
+// AddGroup adds the chunk table of group g of e's finished grouped session.
+func (x *Index) AddGroup(e *Engine, g int) error {
+	if rc := C.mksnap_index_add_group(e.h, x.ix, C.uint32_t(g)); rc != 0 {
+		return fmt.Errorf("mksnap index add group: %s", C.GoString(C.mksnap_last_error(e.h)))
+	}
+	return nil
 }

@@ -81,6 +81,11 @@ class DeltaResult(C.Structure):
                 ("repeat_bytes", C.c_uint64), ("ms_device", C.c_float), ("reserved", C.c_uint32)]
 
 
+class GroupResult(C.Structure):
+    _fields_ = [("n_files", C.c_uint64), ("cdc_bytes", C.c_uint64), ("n_chunks", C.c_uint64), ("n_unique", C.c_uint64),
+                ("first_row", C.c_uint64), ("root", C.c_uint8 * 32)]
+
+
 # every symbol include/mksnap.h declares: (name, restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = [
@@ -112,6 +117,16 @@ SYMBOLS = [
     ("mksnap_index_get", C.c_int, [_P, _P, _P, C.c_uint64]),
     ("mksnap_delta", C.c_int, [_P, _P, C.POINTER(DeltaResult)]),
     ("mksnap_get_chunk_status", C.c_int, [_P, _P, C.c_uint64]),
+    ("mksnap_begin_groups", C.c_int, [_P, C.c_uint32]),
+    ("mksnap_arena_submit_groups", C.c_int, [_P, C.c_int32, C.c_uint64, C.POINTER(Extent), C.c_uint64, _P,
+                                             C.POINTER(Range), C.c_uint64]),
+    ("mksnap_device_submit_groups", C.c_int, [_P, C.c_uint32, C.c_uint64, C.POINTER(Extent), C.c_uint64, _P,
+                                              C.POINTER(Range), C.c_uint64]),
+    ("mksnap_get_group_results", C.c_int, [_P, C.POINTER(GroupResult), C.c_uint32]),
+    ("mksnap_get_group_table", C.c_int, [_P, C.c_uint32, _P, C.c_uint64]),
+    ("mksnap_get_chunk_groups", C.c_int, [_P, _P, C.c_uint64]),
+    ("mksnap_delta_groups", C.c_int, [_P, _P, C.POINTER(DeltaResult), C.c_uint32]),
+    ("mksnap_index_add_group", C.c_int, [_P, _P, C.c_uint32]),
     ("mksnap_comm_unique_id", C.c_int, [_P]),
     ("mksnap_comm_init", C.c_int, [_P, _P, C.c_int32, C.c_int32]),
     ("mksnap_table_rows", C.c_uint64, [_P]),
@@ -177,6 +192,7 @@ class Engine:
         if cdc is not None:
             cfg.cdc = cdc
         self.cfg = cfg
+        self.n_groups = 0  # groups of the current session (0 = ungrouped)
         self.h = _P()
         rc = self.lib.mksnap_create(C.byref(cfg), C.byref(self.h))
         if rc:
@@ -207,6 +223,7 @@ class Engine:
     # -- session -------------------------------------------------------
     def begin(self):
         self._ck(self.lib.mksnap_begin(self.h), "mksnap_begin")
+        self.n_groups = 0
 
     def arena_acquire(self):
         ptr, cap, aid = _P(), C.c_uint64(), C.c_int32()
@@ -240,13 +257,32 @@ class Engine:
         ra = ranges if isinstance(ranges, C.Array) else (Range * max(nr, 1))(*(ranges or []))
         return ea, ne, ra, nr
 
-    def arena_submit(self, arena_id: int, used: int, extents, ranges=None):
-        ea, ne, ra, nr = self._tables(extents, ranges)
-        self._ck(self.lib.mksnap_arena_submit(self.h, arena_id, used, ea, ne, ra, nr), "mksnap_arena_submit")
+    @staticmethod
+    def _groups(groups, ne):
+        import numpy as np
+        g = np.ascontiguousarray(groups, dtype=np.uint32).ravel()
+        if g.size != ne:
+            raise ValueError(f"groups: {g.size} entries for {ne} extents (one per extent)")
+        return g if g.size else np.zeros(1, dtype=np.uint32)
 
-    def device_submit(self, slot: int, used: int, extents, ranges=None):
+    def arena_submit(self, arena_id: int, used: int, extents, ranges=None, groups=None):
+        """groups: one group per extent, in a session started by begin_groups (DESIGN.md section 3c)."""
         ea, ne, ra, nr = self._tables(extents, ranges)
-        self._ck(self.lib.mksnap_device_submit(self.h, slot, used, ea, ne, ra, nr), "mksnap_device_submit")
+        if groups is None:
+            self._ck(self.lib.mksnap_arena_submit(self.h, arena_id, used, ea, ne, ra, nr), "mksnap_arena_submit")
+            return
+        g = self._groups(groups, ne)
+        self._ck(self.lib.mksnap_arena_submit_groups(self.h, arena_id, used, ea, ne, g.ctypes.data, ra, nr),
+                 "mksnap_arena_submit_groups")
+
+    def device_submit(self, slot: int, used: int, extents, ranges=None, groups=None):
+        ea, ne, ra, nr = self._tables(extents, ranges)
+        if groups is None:
+            self._ck(self.lib.mksnap_device_submit(self.h, slot, used, ea, ne, ra, nr), "mksnap_device_submit")
+            return
+        g = self._groups(groups, ne)
+        self._ck(self.lib.mksnap_device_submit_groups(self.h, slot, used, ea, ne, g.ctypes.data, ra, nr),
+                 "mksnap_device_submit_groups")
 
     def device_upload(self, slot: int, dst_off: int, data):
         import numpy as np
@@ -317,6 +353,39 @@ class Engine:
         self._ck(self.lib.mksnap_get_chunk_status(self.h, out.ctypes.data, n), "mksnap_get_chunk_status")
         return out[:n]
 
+    # -- grouped sessions (per-layer tables in one session) -------------
+    def begin_groups(self, n_groups: int):
+        """Start a session whose submits tag every extent with a group in [0, n_groups)."""
+        self._ck(self.lib.mksnap_begin_groups(self.h, n_groups), "mksnap_begin_groups")
+        self.n_groups = n_groups
+
+    def group_results(self, n_groups: int | None = None) -> list:
+        n_groups = self.n_groups if n_groups is None else n_groups
+        out = (GroupResult * max(1, n_groups))()
+        self._ck(self.lib.mksnap_get_group_results(self.h, out, n_groups), "mksnap_get_group_results")
+        return [out[i] for i in range(n_groups)]
+
+    def group_table(self, group: int, n: int):
+        """Group `group`'s sorted-unique table: n rows (its group_results()[group].n_unique)."""
+        import numpy as np
+        t = np.empty((max(n, 1), 32), dtype=np.uint8)
+        self._ck(self.lib.mksnap_get_group_table(self.h, group, t.ctypes.data, n), "mksnap_get_group_table")
+        return t[:n]
+
+    def chunk_groups(self, n: int):
+        """The group of every chunk, uint32 in get_chunks order."""
+        import numpy as np
+        out = np.empty(max(n, 1), dtype=np.uint32)
+        self._ck(self.lib.mksnap_get_chunk_groups(self.h, out.ctypes.data, n), "mksnap_get_chunk_groups")
+        return out[:n]
+
+    def delta_groups(self, ix: "ChunkIndex", n_groups: int | None = None) -> list:
+        """The sequential per-group flow delta -> add_table in one call, ix unchanged: one DeltaResult per group."""
+        n_groups = self.n_groups if n_groups is None else n_groups
+        out = (DeltaResult * max(1, n_groups))()
+        self._ck(self.lib.mksnap_delta_groups(self.h, ix.ix, out, n_groups), "mksnap_delta_groups")
+        return [out[i] for i in range(n_groups)]
+
     # -- multi GPU -----------------------------------------------------
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -377,6 +446,10 @@ class ChunkIndex:
     def add_table(self, eng: Engine):
         """Union with eng's finished session table."""
         eng._ck(self.lib.mksnap_index_add_table(eng.h, self.ix), "mksnap_index_add_table")
+
+    def add_group(self, eng: Engine, group: int):
+        """Union with one group's table of eng's finished grouped session."""
+        eng._ck(self.lib.mksnap_index_add_group(eng.h, self.ix, group), "mksnap_index_add_group")
 
     def get(self, eng: Engine):
         import numpy as np

@@ -6,6 +6,7 @@
 #include "../../include/mksnap.h"
 #include "mksnap_kernels.cuh"
 #include "mksnap_index.cuh"
+#include "mksnap_groups.cuh"
 
 #include <dlfcn.h>
 #include <stdarg.h>
@@ -47,6 +48,7 @@ struct MetaSet {
     CdcFile *d_files = nullptr;
     uint64_t *d_rstart = nullptr, *d_rlen = nullptr;
     uint32_t *d_rstream = nullptr, *d_rflags = nullptr;
+    uint32_t *h_fgroup = nullptr, *d_fgroup = nullptr; // group of each CDC file (grouped sessions; allocated by begin_groups)
     cudaEvent_t ev_done = nullptr; // kernels that read this set have finished
     bool in_flight = false;
 };
@@ -151,6 +153,25 @@ struct mksnap {
     unsigned long long *d_dcnt = nullptr;
     cudaEvent_t ev_delta[2] = {nullptr, nullptr};
     bool delta_done = false; // d_dstatus holds this session's statuses
+
+    // grouped sessions (DESIGN.md section 3c): allocated by the first mksnap_begin_groups, sized for max_chunks
+    uint32_t n_groups = 0;          // 0 = ungrouped session
+    bool groups_ready = false;      // finish built the group tables of this session
+    uint32_t open_group = 0;        // group of the file left open by a MKSNAP_X_MORE extent
+    uint32_t *d_cgroup = nullptr;   // per chunk: its group
+    uint32_t *d_crow = nullptr;     // per chunk: its batch-table row
+    uint64_t *d_gkeys[2] = {nullptr, nullptr}; // (group << rbits) | row, radix double buffer
+    uint8_t *d_gtable = nullptr;    // the group tables, concatenated in group order
+    unsigned long long *d_gfirst = nullptr; // grouped delta: per batch-table row, lowest (group << 32) | chunk
+    unsigned long long *d_gcnt = nullptr;   // grouped delta: 6 counters per group
+    uint32_t *d_gstart = nullptr;   // cstart[G + 1], ustart[G + 1]
+    uint8_t *d_garena = nullptr;    // Merkle nodes of the group tables: rows [0, G) = roots, then inner levels
+    StreamState *d_gss = nullptr;   // stream states of the Merkle launches (all closed; the kernel reads `open`)
+    uint64_t *d_grng = nullptr;     // Merkle ranges: start, len (u64 each), then stream row (u32)
+    uint32_t *d_grflags = nullptr;  // zeros
+    uint64_t garena_rows = 0;
+    std::vector<uint64_t> g_files, g_bytes; // per group, host side
+    std::vector<mksnap_group_result> g_res;
 
     // multi-GPU
     NcclApi nccl;
@@ -692,6 +713,13 @@ void mksnap_destroy(mksnap_t *h)
     cudaFree(h->d_gather); cudaFree(h->d_gcount); cudaFree(h->d_concat);
     cudaFree(h->d_xbounds); cudaFree(h->d_xhdr); cudaFree(h->d_xrec); cudaFree(h->d_xtail);
     cudaFree(h->d_dfirst); cudaFree(h->d_duidx); cudaFree(h->d_ddir); cudaFree(h->d_dstatus); cudaFree(h->d_dcnt);
+    for (auto &m : h->meta) {
+        cudaFreeHost(m.h_fgroup);
+        cudaFree(m.d_fgroup);
+    }
+    cudaFree(h->d_cgroup); cudaFree(h->d_crow); cudaFree(h->d_gkeys[0]); cudaFree(h->d_gkeys[1]); cudaFree(h->d_gtable);
+    cudaFree(h->d_gfirst); cudaFree(h->d_gcnt); cudaFree(h->d_gstart); cudaFree(h->d_garena); cudaFree(h->d_gss);
+    cudaFree(h->d_grng); cudaFree(h->d_grflags);
     for (int i = 0; i < 2; i++)
         if (h->ev_delta[i])
             cudaEventDestroy(h->ev_delta[i]);
@@ -721,6 +749,8 @@ int mksnap_begin(mksnap_t *h)
     h->finished = false;
     h->table_own = false;
     h->delta_done = false;
+    h->n_groups = 0;
+    h->groups_ready = false;
     h->in_session = true;
     return 0;
 }
@@ -778,7 +808,7 @@ int mksnap_get_limits(const mksnap_t *h, mksnap_limits *out)
 }
 
 static int submit_common(mksnap *h, uint32_t slot, uint64_t used, const mksnap_extent *ext, uint64_t n_ext,
-                         const mksnap_range *rng, uint64_t n_rng, HostArena *src)
+                         const mksnap_range *rng, uint64_t n_rng, HostArena *src, const uint32_t *groups = nullptr)
 {
     if (!h->in_session || h->finished)
         return fail(h, MKSNAP_E_STATE, "submit outside begin/finish");
@@ -836,6 +866,8 @@ static int submit_common(mksnap *h, uint32_t slot, uint64_t used, const mksnap_e
             m.h_files[n_files].scratch = big_slots;
             m.h_files[n_files].more_after = more ? x.reserved : 0u;
             m.h_files[n_files].cont = cont ? 1u : 0u;
+            if (groups)
+                m.h_fgroup[n_files] = groups[i];
             if (x.len + (cont ? h->carry_cap : 0) >= SELECT_BIG_FILE) // a continuation is widened by its open chunk on the device
                 big_slots += (x.len + (cont ? h->carry_cap : 0)) / h->prm.min_size + 2;
             cdc_bytes += x.len;
@@ -898,6 +930,10 @@ static int submit_common(mksnap *h, uint32_t slot, uint64_t used, const mksnap_e
     }
     if (n_files)
         CK(h, cudaMemcpyAsync(m.d_files, m.h_files, n_files * sizeof(CdcFile), cudaMemcpyHostToDevice, sc));
+    if (groups && n_files) { // beside the file table: CdcFile itself does not grow
+        CK(h, cudaMemcpyAsync(m.d_fgroup, m.h_fgroup, n_files * 4, cudaMemcpyHostToDevice, sc));
+        h->stats.h2d_bytes += n_files * 4;
+    }
     if (n_rng) {
         CK(h, cudaMemcpyAsync(m.d_rstart, m.h_rstart, n_rng * 8, cudaMemcpyHostToDevice, sc));
         CK(h, cudaMemcpyAsync(m.d_rlen, m.h_rlen, n_rng * 8, cudaMemcpyHostToDevice, sc));
@@ -964,6 +1000,11 @@ static int submit_common(mksnap *h, uint32_t slot, uint64_t used, const mksnap_e
                                                               h->d_chunk_start, h->d_chunk_len, h->d_chunk_end);
             LAUNCH_OK(h);
         }
+        if (groups) {
+            k_group_tag<<<(uint32_t)((n_files + 7) / 8), 256, 0, sk>>>((uint32_t)n_files, m.d_fgroup, h->d_counts, h->d_bases,
+                                                                      h->d_sc, h->max_chunks, h->d_cgroup);
+            LAUNCH_OK(h);
+        }
     }
     CK(h, cudaEventRecord(h->ev[3], sk));
     if (n_files) {
@@ -1026,6 +1067,8 @@ int mksnap_arena_submit(mksnap_t *h, int32_t arena_id, uint64_t used, const mksn
     if (!h)
         return MKSNAP_E_INVAL;
     CK(h, cudaSetDevice(h->cfg.device));
+    if (h->n_groups)
+        return fail(h, MKSNAP_E_STATE, "a grouped session takes mksnap_arena_submit_groups");
     if (arena_id < 0 || (size_t)arena_id >= h->arenas.size() || !h->arenas[arena_id].acquired)
         return fail(h, MKSNAP_E_STATE, "arena %d was not acquired", arena_id);
     if (used > h->cfg.host_arena_bytes)
@@ -1071,6 +1114,8 @@ int mksnap_device_submit(mksnap_t *h, uint32_t slot, uint64_t used, const mksnap
 {
     if (!h || slot >= h->n_slots)
         return MKSNAP_E_INVAL;
+    if (h->n_groups)
+        return fail(h, MKSNAP_E_STATE, "a grouped session takes mksnap_device_submit_groups");
     CK(h, cudaSetDevice(h->cfg.device));
     return submit_common(h, slot, used, extents, n_extents, ranges, n_ranges, nullptr);
 }
@@ -1107,6 +1152,8 @@ int mksnap_sync(mksnap_t *h)
     CK(h, cudaStreamSynchronize(h->s_comp));
     return 0;
 }
+
+static int finish_groups(mksnap *h, uint64_t n, cudaStream_t s); // grouped sessions, below
 
 int mksnap_finish(mksnap_t *h, mksnap_result *out)
 {
@@ -1145,6 +1192,11 @@ int mksnap_finish(mksnap_t *h, mksnap_result *out)
             return rc;
     }
     CK(h, cudaEventRecord(h->ev_fin[2], s));
+    if (h->n_groups) {
+        rc = finish_groups(h, n, s);
+        if (rc)
+            return rc;
+    }
     CK(h, cudaStreamSynchronize(s));
     h->have_fin_times = true;
     memset(out, 0, sizeof *out);
@@ -1159,6 +1211,7 @@ int mksnap_finish(mksnap_t *h, mksnap_result *out)
     h->last_result = *out;
     h->finished = true;
     h->table_own = h->n_ranks == 1;
+    h->groups_ready = h->n_groups != 0;
     return 0;
 }
 
@@ -1475,6 +1528,22 @@ int mksnap_index_get(mksnap_t *h, mksnap_index_t *ix, uint8_t *rows, uint64_t ca
     return 0;
 }
 
+// the delta's buffers, sized for the session: allocated by the first mksnap_delta or mksnap_begin_groups
+static int alloc_delta_buffers(mksnap *h)
+{
+    if (h->d_dstatus)
+        return 0;
+    const uint64_t mc = std::max<uint64_t>(1, h->max_chunks);
+    CK(h, cudaMalloc(&h->d_dfirst, mc * 4));
+    CK(h, cudaMalloc(&h->d_duidx, mc * 4));
+    CK(h, cudaMalloc(&h->d_ddir, ((1ull << mk::dir_bits(mc)) + 1) * 4));
+    CK(h, cudaMalloc(&h->d_dcnt, 6 * sizeof(unsigned long long)));
+    for (int i = 0; i < 2; i++)
+        CK(h, cudaEventCreate(&h->ev_delta[i]));
+    CK(h, cudaMalloc(&h->d_dstatus, mc));
+    return 0;
+}
+
 int mksnap_delta(mksnap_t *h, const mksnap_index_t *ix, mksnap_delta_result *out)
 {
     if (!h || !ix || !out)
@@ -1483,16 +1552,9 @@ int mksnap_delta(mksnap_t *h, const mksnap_index_t *ix, mksnap_delta_result *out
     if (rc)
         return rc;
     CK(h, cudaSetDevice(h->cfg.device));
-    if (!h->d_dstatus) { // first use: the delta's buffers, sized for the session
-        const uint64_t mc = std::max<uint64_t>(1, h->max_chunks);
-        CK(h, cudaMalloc(&h->d_dfirst, mc * 4));
-        CK(h, cudaMalloc(&h->d_duidx, mc * 4));
-        CK(h, cudaMalloc(&h->d_ddir, ((1ull << mk::dir_bits(mc)) + 1) * 4));
-        CK(h, cudaMalloc(&h->d_dcnt, 6 * sizeof(unsigned long long)));
-        CK(h, cudaMalloc(&h->d_dstatus, mc));
-        for (int i = 0; i < 2; i++)
-            CK(h, cudaEventCreate(&h->ev_delta[i]));
-    }
+    rc = alloc_delta_buffers(h);
+    if (rc)
+        return rc;
     cudaStream_t s = h->s_comp;
     const uint64_t n = h->last_result.n_chunks, u = h->n_unique;
     CK(h, cudaEventRecord(h->ev_delta[0], s));
@@ -1546,6 +1608,392 @@ int mksnap_get_chunk_status(mksnap_t *h, uint8_t *status, uint64_t capacity)
         CK(h, cudaMemcpy(status, h->d_dstatus, n, cudaMemcpyDeviceToHost));
     h->stats.d2h_bytes += n;
     return 0;
+}
+
+// ---- grouped sessions (DESIGN.md section 3c) ----------------------------------------------------------------------
+static uint32_t bits_for(uint64_t v) // bits that hold every value in [0, v], at least one
+{
+    uint32_t b = 1;
+    while (b < 64 && (v >> b))
+        ++b;
+    return b;
+}
+
+// allocated once, by the first mksnap_begin_groups; d_cgroup last, so that it marks a complete set
+static int alloc_group_buffers(mksnap *h)
+{
+    if (h->d_cgroup)
+        return 0;
+    int rc = alloc_delta_buffers(h);
+    if (rc)
+        return rc;
+    const uint64_t mx = h->cfg.max_extents, mc = std::max<uint64_t>(1, h->max_chunks);
+    for (auto &m : h->meta) {
+        if (!m.h_fgroup)
+            CK(h, cudaHostAlloc(&m.h_fgroup, mx * 4, cudaHostAllocDefault));
+        if (!m.d_fgroup)
+            CK(h, cudaMalloc(&m.d_fgroup, mx * 4));
+    }
+    // Merkle nodes: G roots, and inner nodes of the groups that have more than 256 rows (fewer than U/64 over all levels)
+    const uint64_t rows = GROUPS_MAX + mc / 64 + 1024;
+    if (!h->d_garena) {
+        CK(h, cudaMalloc(&h->d_crow, mc * 4));
+        for (int k = 0; k < 2; k++)
+            CK(h, cudaMalloc(&h->d_gkeys[k], mc * 8));
+        CK(h, cudaMalloc(&h->d_gtable, mc * 32));
+        CK(h, cudaMalloc(&h->d_gfirst, mc * 8));
+        CK(h, cudaMalloc(&h->d_gcnt, (uint64_t)GROUPS_MAX * 6 * 8));
+        CK(h, cudaMalloc(&h->d_gstart, 2ull * (GROUPS_MAX + 1) * 4));
+        CK(h, cudaMalloc(&h->d_gss, rows * sizeof(StreamState)));
+        CK(h, cudaMemset(h->d_gss, 0, rows * sizeof(StreamState)));
+        CK(h, cudaMalloc(&h->d_grng, rows * 3 * 8));
+        CK(h, cudaMalloc(&h->d_grflags, rows * 4));
+        CK(h, cudaMemset(h->d_grflags, 0, rows * 4));
+        CK(h, cudaMalloc(&h->d_garena, rows * 32));
+        h->garena_rows = rows;
+    }
+    CK(h, cudaMalloc(&h->d_cgroup, mc * 4));
+    return 0;
+}
+
+int mksnap_begin_groups(mksnap_t *h, uint32_t n_groups)
+{
+    if (!h)
+        return MKSNAP_E_INVAL;
+    if (n_groups == 0 || n_groups > GROUPS_MAX)
+        return fail(h, MKSNAP_E_INVAL, "begin_groups: n_groups = %u, must be in [1, %u]", n_groups, GROUPS_MAX);
+    if (h->n_ranks > 1)
+        return fail(h, MKSNAP_E_STATE, "begin_groups: the handle is one rank of %d (grouped sessions are single-rank)", h->n_ranks);
+    CK(h, cudaSetDevice(h->cfg.device));
+    int rc = alloc_group_buffers(h);
+    if (rc)
+        return rc;
+    rc = mksnap_begin(h);
+    if (rc)
+        return rc;
+    h->n_groups = n_groups;
+    h->open_group = 0;
+    h->g_files.assign(n_groups, 0);
+    h->g_bytes.assign(n_groups, 0);
+    h->g_res.clear();
+    return 0;
+}
+
+// a grouped submit is checked whole before anything of the session changes
+static int check_submit_groups(mksnap *h, const mksnap_extent *ext, uint64_t n_ext, const uint32_t *groups)
+{
+    if (!h->n_groups)
+        return fail(h, MKSNAP_E_STATE, "grouped submit in a session that mksnap_begin started (use mksnap_begin_groups)");
+    if (n_ext && (!ext || !groups))
+        return fail(h, MKSNAP_E_INVAL, "grouped submit: null extent or group table");
+    for (uint64_t i = 0; i < n_ext; i++) {
+        if (!(ext[i].flags & MKSNAP_X_CDC))
+            continue;
+        if (groups[i] >= h->n_groups)
+            return fail(h, MKSNAP_E_INVAL, "extent %llu: group %u >= n_groups %u", (unsigned long long)i, groups[i], h->n_groups);
+        if ((ext[i].flags & MKSNAP_X_CONT) && h->open_file && groups[i] != h->open_group)
+            return fail(h, MKSNAP_E_INVAL, "extent %llu: a continuation carries group %u, its file started in group %u",
+                        (unsigned long long)i, groups[i], h->open_group);
+    }
+    return 0;
+}
+
+static void account_groups(mksnap *h, const mksnap_extent *ext, uint64_t n_ext, const uint32_t *groups)
+{
+    for (uint64_t i = 0; i < n_ext; i++) {
+        if (!(ext[i].flags & MKSNAP_X_CDC))
+            continue;
+        h->g_bytes[groups[i]] += ext[i].len;
+        if (!(ext[i].flags & MKSNAP_X_CONT))
+            h->g_files[groups[i]]++;
+        if (ext[i].flags & MKSNAP_X_MORE)
+            h->open_group = groups[i];
+    }
+}
+
+int mksnap_arena_submit_groups(mksnap_t *h, int32_t arena_id, uint64_t used, const mksnap_extent *extents,
+                               uint64_t n_extents, const uint32_t *groups, const mksnap_range *ranges, uint64_t n_ranges)
+{
+    if (!h)
+        return MKSNAP_E_INVAL;
+    int rc = check_submit_groups(h, extents, n_extents, groups);
+    if (rc)
+        return rc;
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (arena_id < 0 || (size_t)arena_id >= h->arenas.size() || !h->arenas[arena_id].acquired)
+        return fail(h, MKSNAP_E_STATE, "arena %d was not acquired", arena_id);
+    if (used > h->cfg.host_arena_bytes)
+        return fail(h, MKSNAP_E_CAPACITY, "used %llu > host arena %llu", (unsigned long long)used,
+                    (unsigned long long)h->cfg.host_arena_bytes);
+    const uint32_t slot = (uint32_t)(h->submit_idx % h->n_slots);
+    rc = submit_common(h, slot, used, extents, n_extents, ranges, n_ranges, &h->arenas[arena_id], groups);
+    if (rc == 0)
+        account_groups(h, extents, n_extents, groups);
+    return rc;
+}
+
+int mksnap_device_submit_groups(mksnap_t *h, uint32_t slot, uint64_t used, const mksnap_extent *extents,
+                                uint64_t n_extents, const uint32_t *groups, const mksnap_range *ranges, uint64_t n_ranges)
+{
+    if (!h || slot >= h->n_slots)
+        return MKSNAP_E_INVAL;
+    int rc = check_submit_groups(h, extents, n_extents, groups);
+    if (rc)
+        return rc;
+    CK(h, cudaSetDevice(h->cfg.device));
+    rc = submit_common(h, slot, used, extents, n_extents, ranges, n_ranges, nullptr, groups);
+    if (rc == 0)
+        account_groups(h, extents, n_extents, groups);
+    return rc;
+}
+
+// Finish of a grouped session, after the batch table and root: chunk -> row, segmented unique over the integer keys
+// (group << rbits) | row, group offsets, then the groups' Merkle levels (one K4 launch per level over all groups)
+static int finish_groups(mksnap *h, uint64_t n, cudaStream_t s)
+{
+    const uint32_t G = h->n_groups;
+    const uint64_t u = h->n_unique;
+    if (n) {
+        const uint32_t tbits = mk::dir_bits(u);
+        k_dir_build<<<grid_for(u + 1, 256), 256, 0, s>>>(h->d_table, (uint32_t)u, tbits, h->d_ddir);
+        LAUNCH_OK(h);
+        const uint32_t rbits = bits_for(u - 1), kbits = rbits + bits_for(G - 1);
+        k_group_keys<<<grid_for(n, 256), 256, 0, s>>>(h->d_digests, (uint32_t)n, mk::RowSet{h->d_table, h->d_ddir, (uint32_t)u, tbits},
+                                                      h->d_cgroup, rbits, h->d_crow, h->d_gkeys[0]);
+        LAUNCH_OK(h);
+        // exact keys: only the 8-bit digits the keys use, and no tie fix (K3's session scratch is free after the batch table)
+        const uint32_t nblocks = (uint32_t)((n + SORT_TILE - 1) / SORT_TILE);
+        int cur = 0;
+        for (uint32_t shift = 0; shift < kbits; shift += 8) {
+            k_radix_hist<<<nblocks, SORT_THREADS, 0, s>>>(h->d_gkeys[cur], n, (int)shift, h->d_hist, nblocks);
+            LAUNCH_OK(h);
+            int rc = scan_u32(h, h->d_hist, h->d_hist, (uint64_t)256 * nblocks, s);
+            if (rc)
+                return rc;
+            k_radix_scatter<<<nblocks, SORT_THREADS, 0, s>>>(h->d_gkeys[cur], h->d_idx[0], n, (int)shift, h->d_hist, nblocks,
+                                                             h->d_gkeys[cur ^ 1], h->d_idx[1]); // payload unused
+            LAUNCH_OK(h);
+            cur ^= 1;
+        }
+        const uint64_t *keys = h->d_gkeys[cur];
+        k_group_flags<<<grid_for(n, 256), 256, 0, s>>>(keys, (uint32_t)n, h->d_flags);
+        LAUNCH_OK(h);
+        int rc = scan_u32(h, h->d_flags, h->d_pos, n, s);
+        if (rc)
+            return rc;
+        k_group_compact<<<grid_for(2 * n, 256), 256, 0, s>>>(keys, h->d_flags, h->d_pos, (uint32_t)n, rbits, h->d_table, h->d_gtable);
+        LAUNCH_OK(h);
+        k_group_bounds<<<grid_for(n + 1, 256), 256, 0, s>>>(keys, h->d_flags, h->d_pos, (uint32_t)n, rbits, G, h->d_gstart,
+                                                           h->d_gstart + G + 1);
+        LAUNCH_OK(h);
+    } else {
+        CK(h, cudaMemsetAsync(h->d_gstart, 0, 2ull * (G + 1) * 4, s));
+    }
+    std::vector<uint32_t> st(2ull * (G + 1));
+    CK(h, cudaMemcpyAsync(st.data(), h->d_gstart, st.size() * 4, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s));
+    h->stats.d2h_bytes += st.size() * 4;
+    const uint32_t *cstart = st.data(), *ustart = st.data() + G + 1;
+
+    // Merkle plan on the host (the same rule as merkle_from, per group): a level hashes every group that does not yet
+    // have one digest -- at level 0 every group, so an empty group gets SHA256("") and a one-row group SHA256(row).  A
+    // group whose level yields one node writes it to its root row g; otherwise its nodes go to fresh rows after the roots.
+    std::vector<uint64_t> at(G), cnt(G), rs, rl;
+    std::vector<uint32_t> sid, active(G), keep;
+    std::vector<std::pair<size_t, size_t>> levels;
+    for (uint32_t g = 0; g < G; g++) {
+        at[g] = ustart[g];
+        cnt[g] = ustart[g + 1] - ustart[g];
+        active[g] = g;
+    }
+    uint64_t next_row = G;
+    while (!active.empty()) {
+        const size_t b = rs.size();
+        keep.clear();
+        for (uint32_t g : active) {
+            const uint64_t c = cnt[g], nout = c == 0 ? 1 : (c + 255) / 256;
+            if (nout == 1) {
+                rs.push_back(at[g] * 32);
+                rl.push_back(c * 32);
+                sid.push_back(g);
+                continue;
+            }
+            for (uint64_t j = 0; j < nout; j++) {
+                rs.push_back((at[g] + 256 * j) * 32);
+                rl.push_back(std::min<uint64_t>(256, c - 256 * j) * 32);
+                sid.push_back((uint32_t)(next_row + j));
+            }
+            at[g] = next_row;
+            cnt[g] = nout;
+            next_row += nout;
+            keep.push_back(g);
+        }
+        levels.emplace_back(b, rs.size());
+        active.swap(keep);
+    }
+    const uint64_t R = h->garena_rows;
+    if (next_row > R || rs.size() > R)
+        return fail(h, MKSNAP_E_CAPACITY, "group Merkle plan: %llu nodes exceed %llu rows", (unsigned long long)next_row,
+                    (unsigned long long)R);
+    uint64_t *d_start = h->d_grng, *d_len = h->d_grng + R;
+    uint32_t *d_sid = reinterpret_cast<uint32_t *>(h->d_grng + 2 * R);
+    CK(h, cudaMemcpyAsync(d_start, rs.data(), rs.size() * 8, cudaMemcpyHostToDevice, s));
+    CK(h, cudaMemcpyAsync(d_len, rl.data(), rl.size() * 8, cudaMemcpyHostToDevice, s));
+    CK(h, cudaMemcpyAsync(d_sid, sid.data(), sid.size() * 4, cudaMemcpyHostToDevice, s));
+    h->stats.h2d_bytes += rs.size() * 20;
+    for (size_t lv = 0; lv < levels.size(); lv++) {
+        const size_t b = levels[lv].first, m = levels[lv].second - b;
+        CK(h, cudaMemsetAsync(&h->d_sc->work, 0, 4, s));
+        k_sha256_streams<<<(uint32_t)std::min<uint64_t>((m + 31) / 32, (uint64_t)h->sm_count * 4), SS_THREADS, 0, s>>>(
+            lv == 0 ? h->d_gtable : h->d_garena, d_start + b, d_len + b, (uint32_t)m, d_sid + b, h->d_grflags, h->d_gss,
+            h->d_garena, &h->d_sc->work, 32u, 1u);
+        LAUNCH_OK(h);
+    }
+    std::vector<uint8_t> roots(32ull * G);
+    CK(h, cudaMemcpyAsync(roots.data(), h->d_garena, roots.size(), cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s)); // the plan vectors are read by the copies above until here
+    h->stats.d2h_bytes += roots.size();
+    h->g_res.assign(G, mksnap_group_result{});
+    for (uint32_t g = 0; g < G; g++) {
+        mksnap_group_result &r = h->g_res[g];
+        r.n_files = h->g_files[g];
+        r.cdc_bytes = h->g_bytes[g];
+        r.n_chunks = cstart[g + 1] - cstart[g];
+        r.n_unique = ustart[g + 1] - ustart[g];
+        r.first_row = ustart[g];
+        memcpy(r.root, roots.data() + 32ull * g, 32);
+    }
+    return 0;
+}
+
+static int group_check(mksnap *h, const char *what)
+{
+    if (!h->n_groups)
+        return fail(h, MKSNAP_E_STATE, "%s: the session is not grouped (mksnap_begin_groups)", what);
+    if (!h->finished || !h->groups_ready)
+        return fail(h, MKSNAP_E_STATE, "%s needs a finished grouped session", what);
+    return 0;
+}
+
+int mksnap_get_group_results(mksnap_t *h, mksnap_group_result *out, uint32_t n_groups)
+{
+    if (!h || !out)
+        return MKSNAP_E_INVAL;
+    int rc = group_check(h, "get_group_results");
+    if (rc)
+        return rc;
+    if (n_groups != h->n_groups)
+        return fail(h, MKSNAP_E_INVAL, "get_group_results: n_groups %u, the session has %u", n_groups, h->n_groups);
+    memcpy(out, h->g_res.data(), n_groups * sizeof(mksnap_group_result));
+    return 0;
+}
+
+int mksnap_get_group_table(mksnap_t *h, uint32_t group, uint8_t *rows, uint64_t capacity_rows)
+{
+    if (!h)
+        return MKSNAP_E_INVAL;
+    int rc = group_check(h, "get_group_table");
+    if (rc)
+        return rc;
+    if (group >= h->n_groups)
+        return fail(h, MKSNAP_E_INVAL, "get_group_table: group %u >= n_groups %u", group, h->n_groups);
+    const mksnap_group_result &r = h->g_res[group];
+    if (r.n_unique > capacity_rows || (r.n_unique && !rows))
+        return fail(h, MKSNAP_E_CAPACITY, "get_group_table: need %llu rows", (unsigned long long)r.n_unique);
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (r.n_unique)
+        CK(h, cudaMemcpy(rows, h->d_gtable + r.first_row * 32, r.n_unique * 32, cudaMemcpyDeviceToHost));
+    h->stats.d2h_bytes += r.n_unique * 32;
+    return 0;
+}
+
+int mksnap_get_chunk_groups(mksnap_t *h, uint32_t *groups, uint64_t capacity)
+{
+    if (!h)
+        return MKSNAP_E_INVAL;
+    int rc = group_check(h, "get_chunk_groups");
+    if (rc)
+        return rc;
+    const uint64_t n = h->last_result.n_chunks;
+    if (n > capacity || (n && !groups))
+        return fail(h, MKSNAP_E_CAPACITY, "get_chunk_groups: need %llu entries", (unsigned long long)n);
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (n)
+        CK(h, cudaMemcpy(groups, h->d_cgroup, n * 4, cudaMemcpyDeviceToHost));
+    h->stats.d2h_bytes += n * 4;
+    return 0;
+}
+
+int mksnap_delta_groups(mksnap_t *h, const mksnap_index_t *ix, mksnap_delta_result *out, uint32_t n_groups)
+{
+    if (!h || !ix || !out)
+        return MKSNAP_E_INVAL;
+    int rc = own_table_check(h, ix, "delta_groups");
+    if (rc)
+        return rc;
+    if ((rc = group_check(h, "delta_groups")))
+        return rc;
+    const uint32_t G = h->n_groups;
+    if (n_groups != G)
+        return fail(h, MKSNAP_E_INVAL, "delta_groups: n_groups %u, the session has %u", n_groups, G);
+    CK(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t s = h->s_comp;
+    const uint64_t n = h->last_result.n_chunks, u = h->n_unique;
+    CK(h, cudaEventRecord(h->ev_delta[0], s));
+    CK(h, cudaMemsetAsync(h->d_gcnt, 0, (uint64_t)G * 6 * 8, s));
+    if (n) {
+        // each unique batch row is looked up in the index once; chunks only claim their row
+        k_gdelta_rows<<<grid_for(u, 256), 256, 0, s>>>(h->d_table, (uint32_t)u, index_view(ix), h->d_gfirst);
+        LAUNCH_OK(h);
+        k_gdelta_first<<<grid_for(n, 256), 256, 0, s>>>(h->d_crow, h->d_cgroup, (uint32_t)n, h->d_gfirst);
+        LAUNCH_OK(h);
+        const uint32_t grid = (uint32_t)std::min<uint64_t>(grid_for(n, DELTA_THREADS), (uint64_t)h->sm_count * 8);
+        if (G <= GD_SMEM_GROUPS)
+            k_gdelta_classify<true><<<grid, DELTA_THREADS, 0, s>>>((uint32_t)n, h->d_crow, h->d_cgroup, h->d_gfirst, h->d_chunk_len,
+                                                                  G, h->d_dstatus, h->d_gcnt);
+        else
+            k_gdelta_classify<false><<<grid, DELTA_THREADS, 0, s>>>((uint32_t)n, h->d_crow, h->d_cgroup, h->d_gfirst,
+                                                                   h->d_chunk_len, G, h->d_dstatus, h->d_gcnt);
+        LAUNCH_OK(h);
+    }
+    CK(h, cudaEventRecord(h->ev_delta[1], s));
+    std::vector<unsigned long long> c((uint64_t)G * 6);
+    CK(h, cudaMemcpyAsync(c.data(), h->d_gcnt, c.size() * 8, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s));
+    h->stats.d2h_bytes += c.size() * 8;
+    float ms = 0;
+    CK(h, cudaEventElapsedTime(&ms, h->ev_delta[0], h->ev_delta[1]));
+    for (uint32_t g = 0; g < G; g++) {
+        mksnap_delta_result &o = out[g];
+        memset(&o, 0, sizeof o);
+        const unsigned long long *x = c.data() + 6ull * g;
+        o.index_rows = ix->n;
+        o.known_chunks = x[0];
+        o.new_chunks = x[1];
+        o.repeat_chunks = x[2];
+        o.known_bytes = x[3];
+        o.new_bytes = x[4];
+        o.repeat_bytes = x[5];
+        o.ms_device = ms;
+    }
+    h->delta_done = true;
+    return 0;
+}
+
+int mksnap_index_add_group(mksnap_t *h, mksnap_index_t *ix, uint32_t group)
+{
+    if (!h || !ix)
+        return MKSNAP_E_INVAL;
+    int rc = own_table_check(h, ix, "index_add_group");
+    if (rc)
+        return rc;
+    if ((rc = group_check(h, "index_add_group")))
+        return rc;
+    if (group >= h->n_groups)
+        return fail(h, MKSNAP_E_INVAL, "index_add_group: group %u >= n_groups %u", group, h->n_groups);
+    CK(h, cudaSetDevice(h->cfg.device));
+    const mksnap_group_result &r = h->g_res[group];
+    return r.n_unique ? index_union(h, ix, h->d_gtable + r.first_row * 32, r.n_unique, false) : 0;
 }
 
 #include "mksnap_comm.inc"

@@ -198,6 +198,7 @@ MKHOST_SCAN_CONTENT = 4   # content-aware AddLayerByScan (implies FILE_DIGESTS)
 MKHOST_MATERIALIZE = 8    # commit_copy_ops also performs the copy onto the file system, from the arena
 MKHOST_MATERIALIZE_CHOWN = 16
 MKHOST_UNTAR = 32         # UpdateFromTarReader(untar=true): also write the members under the root
+MKHOST_LAYER_TABLES = 64  # commit_layers: per-layer chunk tables (a grouped engine session, layer i = group i)
 MKHOST_COPY_CHOWN, MKHOST_COPY_INTERNAL, MKHOST_COPY_PRESERVE_OWNER, MKHOST_COPY_DEFERRED = 1, 2, 4, 8
 
 
@@ -264,10 +265,14 @@ class MemFS:
         return _layer_dict(out)
 
     def commit_layers(self, eng: abi.Engine, now_unix: int, layers: Sequence[Sequence[CopyOperation]], n_threads: int = 0,
-                      tar_fds: Optional[Sequence[int]] = None, flags: int = 0):
-        """Consecutive layers of one build in ONE engine session (all TarDigest chains advance together)."""
+                      tar_fds: Optional[Sequence[int]] = None, flags: int = 0, layer_tables: bool = False):
+        """Consecutive layers of one build in ONE engine session (all TarDigest chains advance together).  root /
+        n_chunks / n_unique describe the whole batch, or with layer_tables=True each layer's own chunk table; the
+        grouped session then stays open on eng for delta_groups / group_table / ChunkIndex.add_group."""
         err = C.create_string_buffer(1024)
         n = len(layers)
+        if layer_tables:
+            flags |= MKHOST_LAYER_TABLES
         specs, keep, outs = (LayerSpec * max(1, n))(), [], (LayerResult * max(1, n))()
         for i, ops in enumerate(layers):
             arr, k = _ops(ops)
@@ -276,6 +281,7 @@ class MemFS:
             specs[i].tar_fd = tar_fds[i] if tar_fds is not None else -1
         if load().mkhost_memfs_commit_layers(self.h, eng.h, now_unix, specs, n, n_threads, flags, outs, err, len(err)):
             raise HostError(err.value.decode())
+        eng.n_groups = n if flags & MKHOST_LAYER_TABLES else 0
         return [_layer_dict(outs[i]) for i in range(n)]
 
     def file_digest(self, dst: str) -> Optional[bytes]:

@@ -262,8 +262,8 @@ int mkhost_memfs_commit_layers(mkhost_memfs *m, mksnap_t *eng, int64_t now_unix,
     try {
         if (!m || !eng || (!specs && n_layers) || (!outs && n_layers))
             throw HostError("null argument");
-        if (flags & ~(uint32_t)MKHOST_NO_TAR_DIGEST)
-            throw HostError("commit layers: only MKHOST_NO_TAR_DIGEST is supported for a batch");
+        if (flags & ~(uint32_t)(MKHOST_NO_TAR_DIGEST | MKHOST_LAYER_TABLES))
+            throw HostError("commit layers: only MKHOST_NO_TAR_DIGEST and MKHOST_LAYER_TABLES are supported for a batch");
         m->fs.set_now(now_unix);
         // the layer maps are built in order -- each AddLayerByCopyOps sees the tree its predecessors left
         // (mem_fs.go:276-289) -- and only then packed together
